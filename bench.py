@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — env agent-steps/s of the vectorised QuadSwarm env step on B200 (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--config c2|c3|c4] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--config c2|c3|c4] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one control step (2 physics sub-steps + collisions + observations, auto-reset included) of every env
 of the workload.  Default workload = BASELINE.json configs[2] ("c3"): 8 drones x 4096 envs PER GPU (weak scaling),
@@ -410,11 +410,13 @@ class StepRunner:
         self.eng.close()
 
 
-def time_blocks(torch, dist, runner, K, R, world, side=None, metrics=None, gather_every=100):
+def time_blocks(torch, dist, runner, K, R, world, side=None, metrics=None, gather_every=100, lead=0):
     """R back-to-back blocks of exactly K control steps, each bracketed by its own pair of CUDA events on the launching
-    stream.  Returns the (start, end) event pairs.  The optional cross-GPU metrics gather (NCCL all-reduce of a small
-    vector every `gather_every` steps) runs on a side stream that only WAITS for the step stream — it is never an edge of
-    the step chain — and is joined after the last block."""
+    stream, behind `lead` untimed steps enqueued without a synchronise in between: they keep the device busy while the
+    host enqueues the first block, so no launch latency falls inside it.  Returns the (start, end) event pairs and
+    leaves the ring slot of the last timed step in runner.last_slot.  The optional cross-GPU metrics gather (NCCL
+    all-reduce of a small vector every `gather_every` steps) runs on a side stream that only WAITS for the step stream —
+    it is never an edge of the step chain — and is joined after the last block."""
     st = runner.stream
     pairs = []
     since = 0
@@ -424,11 +426,13 @@ def time_blocks(torch, dist, runner, K, R, world, side=None, metrics=None, gathe
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize()
+        runner.run(lead)
         for b in range(R):
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record(st)
             runner.run(K)
             e1.record(st)
+            runner.last_slot = (runner.counter - 1) % runner.P
             pairs.append((e0, e1))
             since += K
             if side is not None and since >= gather_every:
@@ -456,8 +460,10 @@ def block_times(torch, dist, pairs, world, dev):
     return ms
 
 
-def measure_workload(torch, dist, name, args, local_rank, rank, world, K, target_s, clocks=None, side=None, metrics=None, wrapped=False):
-    """Device-resident agent-steps/s of one workload: R blocks of K chained step launches, median block."""
+def measure_workload(torch, dist, name, args, local_rank, rank, world, K, target_s=None, clocks=None, side=None, metrics=None, wrapped=False):
+    """Device-resident agent-steps/s of one workload.  target_s None: one timed window of exactly K chained step
+    launches.  Otherwise R blocks of K, R chosen from two pilot blocks so that about target_s seconds are timed, median
+    block."""
     cfg = CONFIGS[name]
     E = (args.envs if name == args.config and args.envs else cfg['E'])
     runner = StepRunner(torch, cfg, E, args, local_rank, rank, K, graph=not args.no_graph, stagger=not args.lockstep, wrapped=wrapped)
@@ -466,10 +472,14 @@ def measure_workload(torch, dist, name, args, local_rank, rank, world, K, target
         runner.run(max(3, args.warmup))
         runner.align()
         runner.stream.synchronize()
-    # pilot blocks: estimate the block time, warm the graphs
-    evp = time_blocks(torch, dist, runner, K, 2, world)
-    est_ms = max(1e-3, evp[1][0].elapsed_time(evp[1][1]))
-    R = int(min(5000, max(1, np.ceil(target_s * 1e3 / est_ms))))
+    if target_s is None:
+        # the lead-in walks the whole ring once: every graph has been replayed (uploaded) before the window
+        R, lead = 1, runner.P
+    else:
+        # pilot blocks: estimate the block time, warm the graphs
+        evp = time_blocks(torch, dist, runner, K, 2, world)
+        est_ms = max(1e-3, evp[1][0].elapsed_time(evp[1][1]))
+        R, lead = int(min(5000, max(1, np.ceil(target_s * 1e3 / est_ms)))), 0
     if world > 1:
         t = torch.tensor([R], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -483,7 +493,7 @@ def measure_workload(torch, dist, name, args, local_rank, rank, world, K, target
     if clocks is not None:
         clocks.start()
     K_eff = K
-    pairs = time_blocks(torch, dist, runner, K, R, world, side=side, metrics=metrics)
+    pairs = time_blocks(torch, dist, runner, K, R, world, side=side, metrics=metrics, lead=lead)
     clk = clocks.stop() if clocks is not None else None
     ms = block_times(torch, dist, pairs, world, dev)
     if runner.eng.handover_timeouts:
@@ -500,6 +510,24 @@ def measure_workload(torch, dist, name, args, local_rank, rank, world, K, target
                ring_mb=dict(actions=runner.P * A * 16 / 1e6, observations=runner.P * A * D * 4 / 1e6), graphs=runner.NG,
                steps_per_graph=runner.Kg)
     return res
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(torch, runner, out_dir):
+    """What the last timed step returned to its caller (observations, rewards, dones of every env of this rank) as
+    float32 DIR/<name>.npy.  Above DUMP_BYTES in all, the same fixed sample of envs (seeded, in env order) of each."""
+    k = runner.last_slot
+    out = dict(observations=runner.obs[k], rewards=runner.rew[k], dones=runner.done[k])
+    per_env = 4 * sum(v[0].numel() for v in out.values())
+    if per_env * runner.E > DUMP_BYTES:
+        keep = np.sort(np.random.RandomState(0).choice(runner.E, DUMP_BYTES // per_env, replace=False))
+        idx = torch.from_numpy(keep).to(runner.dev)
+        out = {name: v.index_select(0, idx) for name, v in out.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, f'{name}.npy'), v.float().cpu().numpy())
 
 
 def run_cuda_arm(args):
@@ -521,9 +549,11 @@ def run_cuda_arm(args):
     side = torch.cuda.Stream(device=dev) if world > 1 else None
     metrics = torch.zeros(64, device=dev) if world > 1 else None
     clocks = ClockSampler(local_rank) if rank == 0 else None
-    main = measure_workload(torch, dist, args.config, args, local_rank, rank, world, K, args.target_seconds, clocks=clocks,
+    main = measure_workload(torch, dist, args.config, args, local_rank, rank, world, K, clocks=clocks,
                             side=side, metrics=metrics, wrapped=args.wrapped_main)
     runner = main['runner']
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, runner, args.dump_outputs)
     E, N, A, D, M = main['E'], main['N'], main['A'], main['D'], main['M']
     gathers = int(metrics[1].item()) if metrics is not None else 0
     runner.close()
@@ -705,10 +735,9 @@ def run_cuda_arm(args):
             'warmup': args.warmup, 'ms_per_step': main['med_ms'] / K, 'higher_is_better': True, 'scaling': 'weak',
             'vs_baseline': None, 'dtype': 'f32', 'data': 'synthetic',
             'config': conf,
-            'timing': {'protocol': (f'{main["blocks"]} back-to-back blocks of exactly {K} control steps, each block bracketed by CUDA events on the '
-                                    f'launching stream; value / ms_per_step are the MEDIAN block (max over ranks per block)'),
-                       'blocks': main['blocks'], 'block_ms_median': main['med_ms'], 'block_ms_min': main['block_ms_min'],
-                       'block_ms_max': main['block_ms_max'],
+            'timing': {'protocol': (f'one window of exactly {K} control steps bracketed by CUDA events on the launching stream, enqueued '
+                                    f'behind {main["ring_slots"]} untimed steps; value / ms_per_step are that window (max over ranks)'),
+                       'window_ms': main['med_ms'],
                        'episodes': ('generated on the device at every auto-reset' if dev_scn else 'host-generated tables, uploaded once'),
                        'auto_resets': ('envs start at staggered ticks: every control step carries E / (ep_len + 1) auto-resets' if not args.lockstep
                                        else 'envs in lock-step: all envs reset in the same step every ep_len + 1 steps'),
@@ -760,11 +789,12 @@ def main():
     ap.add_argument('--wrapped-main', action='store_true', help='tuning: time the headline workload WITH the training wrappers (the line is then not the BASELINE metric)')
     ap.add_argument('--no-extras', action='store_true', help='skip the rollout / large-batch explanatory measurements')
     ap.add_argument('--lockstep', action='store_true', help='start all envs at tick 0 (all auto-resets fall into the same step)')
-    ap.add_argument('--target-seconds', type=float, default=0.5,
-                    help='repeat the K-step block until about this much time is measured (the clock sampler needs load)')
     ap.add_argument('--no-graph', action='store_true')
     ap.add_argument('--host-tables', action='store_true', help='use host-generated episode tables even where a device generator exists')
     ap.add_argument('--no-cpu-baseline', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write the observations / rewards / dones of the last timed step (rank 0) '
+                         'as float32 DIR/<name>.npy, at most 64 MB in all (a fixed sample of envs beyond that)')
     args = ap.parse_args()
     if args.impl == 'reference':
         run_reference_arm(args)

@@ -59,11 +59,12 @@ def _plants_room(rs):
 
 
 CASES = [
-    # name, env kwargs, T steps, seeds, planted states, obs stride in the fixture
+    # name, env kwargs, T steps, seeds, planted states, obs stride in the fixture, state-snapshot stride (default: the
+    # obs stride; 2 where every-step snapshots would take the fixture past 1 MB)
     dict(name='single_1', kw=dict(num_agents=1, neighbor_visible_num=0, neighbor_obs_type='none', ep_time=1.0,
                                   quads_mode='static_same_goal'), T=230, seed=11, obs_stride=1),
     dict(name='c2_same_goal_8', kw=dict(num_agents=8, neighbor_visible_num=6, ep_time=1.0,
-                                        quads_mode='static_same_goal'), T=230, seed=21, obs_stride=1),
+                                        quads_mode='static_same_goal'), T=230, seed=21, obs_stride=1, state_stride=2),
     dict(name='all_neighbors_8', kw=dict(num_agents=8, neighbor_visible_num=-1, ep_time=0.6,
                                          quads_mode='static_diff_goal', obs_repr='xyz_vxyz_R_omega_wall'),
          T=130, seed=31, obs_stride=1),
@@ -77,7 +78,7 @@ CASES = [
                                         rew_coeff=dict(pos=1.0, effort=0.05, spin=0.1, vel=0.0, crash=1.0, orient=1.0,
                                                        yaw=0.0, quadcol_bin=5.0, quadcol_bin_smooth_max=4.0,
                                                        quadcol_bin_obst=5.0)),
-         T=230, seed=61, obs_stride=1, plant='obst', plant_at=[5, 120]),
+         T=230, seed=61, obs_stride=1, state_stride=2, plant='obst', plant_at=[5, 120]),
     dict(name='c4_swarm_vs_swarm_16', kw=dict(num_agents=16, neighbor_visible_num=6, ep_time=4.5,
                                               quads_mode='swarm_vs_swarm'), T=500, seed=71, obs_stride=10),
     dict(name='dynamic_formations_8', kw=dict(num_agents=8, neighbor_visible_num=6, ep_time=0.8,
@@ -221,9 +222,9 @@ def run_reference_case(case):
                dyn_t=np.array([t for t, _ in dyn_log], dtype=int), dyn_rows=np.array([r for _, r in dyn_log]),
                obst_t=np.array([t for t, _ in obst_log], dtype=int),
                obst_xy=np.array([o for _, o in obst_log]),
-               case_json=np.array(json.dumps(dict(name=case['name'], kw=kw, T=T, seed=seed,
-                                                  obs_stride=case['obs_stride'], D=int(D)))))
-    stride = max(1, case['obs_stride'])
+               case_json=np.array(json.dumps(dict(name=case['name'], kw=kw, T=T, seed=seed, obs_stride=case['obs_stride'],
+                                                  state_stride=case.get('state_stride', case['obs_stride']), D=int(D)))))
+    stride = max(1, case.get('state_stride', case['obs_stride']))
     for k in state_keys:
         arr = np.array(states[k])
         out['state_' + k] = arr[::stride]

@@ -7,6 +7,8 @@ in this order: $QS_REFERENCE_ROOT, oracle/_ref (a `pip install --target` of the 
 Nothing here is imported by the product package.
 """
 import os
+import shutil
+import stat
 import sys
 import contextlib
 import io
@@ -14,11 +16,35 @@ import io
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
+_MIRROR = os.path.join(_HERE, '_ref')
+MIRROR_PACKAGES = ('gym_art', 'swarm_rl')
 
 
-def reference_root():
+def mirror_reference():
+    """Mirror the reference's two python packages into oracle/_ref (git-ignored), so that a copy of this tree taken to
+    a machine without the reference still runs it (bench.py's CPU arms).  The source is the reference tree
+    `reference_root()` finds other than the mirror itself; without one, an existing mirror is kept.  The trees are
+    copied as they are: `pip install --target` of the reference drops its namespace sub-packages, e.g.
+    scenarios/obstacles."""
+    src = reference_root(mirror=False)
+    if src is None:
+        return
+    for pkg in MIRROR_PACKAGES:
+        target = os.path.join(_MIRROR, pkg)
+        if os.path.isdir(target):
+            # copytree keeps the modes of a read-only checkout; without write permission on its directories the
+            # previous mirror could not be removed by anyone but root
+            for dirpath, _, _ in os.walk(target):
+                os.chmod(dirpath, os.stat(dirpath).st_mode | stat.S_IWUSR)
+            shutil.rmtree(target)
+        shutil.copytree(os.path.join(src, pkg), target,
+                        ignore=shutil.ignore_patterns('*.gif', '*.png', '*.pdf', '__pycache__', '*.pyc'))
+
+
+def reference_root(mirror=True):
+    """The first reference tree in the order of the module docstring; mirror=False passes over oracle/_ref."""
     for cand in (os.environ.get('QS_REFERENCE_ROOT'), os.path.join(_HERE, '_ref'), '/root/reference'):
-        if cand and os.path.isdir(os.path.join(cand, 'gym_art', 'quadrotor_multi')):
+        if cand and (mirror or os.path.abspath(cand) != _MIRROR) and os.path.isdir(os.path.join(cand, 'gym_art', 'quadrotor_multi')):
             return cand
     return None
 
